@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]             # headline: C2, weak scaling
     python bench.py --workload {c1,c2,c3,c4,c5} [--scaling {weak,strong}] [...]
     python bench.py --impl reference [...]                          # the reference's CPU path
+    python bench.py --dump-outputs DIR [...]                        # also write the results (.npy)
 
 Workloads (SURVEY §8d; inputs are the reference benchmarks' own, generated in HBM by
 b200_synthetic_generators_device):
@@ -24,6 +25,12 @@ additions (SURVEY §8e). c4 shards by column: no exchange at all.
 With no --workload the headline line (c2, weak) also carries an "extras" object: short runs of the
 other BASELINE configs at this N (N = 1: c3, the per-GPU shares of c4 and c5, pageable-memory e2e, the
 reference's own GPU kernels on the same inputs; N > 1: strong-scaling c2, c4, c5).
+
+--dump-outputs DIR writes, on rank 0, what the last timed device-resident step of the measured
+workload returned, so that two builds can be compared output for output (the inputs depend only on
+the arguments): DIR/commitments.npy (c1-c4: the commitment of every column) or
+DIR/projective_results.npy (c5: the projective MSM result), float64 [columns, bytes] holding the
+specified bytes of each result, one byte value per element.
 """
 import argparse
 import ctypes as C
@@ -409,6 +416,16 @@ def run_workload(env, name, scaling, steps, warmup, with_e2e=True, sampler=None)
     return res
 
 
+def dump_outputs(directory, st):
+    """The device-resident result of the last timed step as float64 byte values (see the module
+    docstring); struct padding is left out."""
+    from tests import common
+    os.makedirs(directory, exist_ok=True)
+    k = st["dev_result"].shape[1] if st["fixed"] else common.CMP[st["curve"]]
+    name = "projective_results" if st["fixed"] else "commitments"
+    np.save(os.path.join(directory, name + ".npy"), st["dev_result"][:, :k].astype(np.float64))
+
+
 def release(res):
     st = res.pop("_state", None)
     return st
@@ -441,6 +458,8 @@ def run_cuda(args, rank, local_rank, world):
     clocks = sampler.stop() if rank == 0 else None
     st = release(main)
     curve = st["curve"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, st)
 
     extras = {}
     cpu, cpu_same = None, None
@@ -586,7 +605,11 @@ def main():
     ap.add_argument("--scaling", default=None, choices=["weak", "strong"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step to DIR as .npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

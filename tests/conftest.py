@@ -21,15 +21,6 @@ def port():
 
 
 @pytest.fixture(scope="session")
-def refcpu():
-    """The reference's own CPU path (oracle/_ref), when the prebuilt library is present."""
-    from oracle import refcpu as r
-    if not r.available():
-        pytest.skip("oracle/_ref/libblitzar_ref_cpu.so not built")
-    return r
-
-
-@pytest.fixture(scope="session")
 def emul():
     """CPU emulation of the product's kernel bodies (tests/emul) — test infrastructure."""
     from tests.emul import harness

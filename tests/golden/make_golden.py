@@ -1,7 +1,9 @@
 """Generates the committed golden fixtures from the REFERENCE's own CPU implementation
-(oracle/_ref, built from /root/reference by oracle/ref_build/Makefile). Run in the build container:
+(oracle/_ref, built from the reference's sources by oracle/ref_build/Makefile):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [fixture ...] [--out DIR]
+
+(default fixture: commit). `ref_gpu` runs the reference's GPU kernels and so needs a B200.
 
 Inputs are seeded; generators for the Weierstrass curves come from the reference's
 fast_random_number_generator{i+1,i+2} -> generate_random_element scheme
@@ -52,10 +54,6 @@ def main():
                         compressed=refcpu.normalize(0, g))
 
 
-if __name__ == "__main__":
-    main()
-
-
 def make_inner_product_fixture():
     """tests/golden/inner_product.npz: proofs produced by the reference's cpu backend
     (sxt_curve25519_prove_inner_product semantics) for n = 1, 2, 5, 16, 37 with a transcript
@@ -84,3 +82,139 @@ def make_inner_product_fixture():
     out["num_cases"] = len(cases)
     out["generators_offset"] = 11
     np.savez_compressed(os.path.join(HERE, "inner_product.npz"), **out)
+
+
+def make_oracle_cases_fixture():
+    """tests/golden/oracle_cases.npz: the reference's commitments, fixed-base MSMs and normalisation
+    on the seeded cases of tests/test_oracle.py."""
+    from oracle import port
+    from tests import common, test_oracle
+    assert refcpu.commit(0, common.golden_columns()).tolist() == common.GOLDEN_COMMITMENTS
+    out = {}
+    for curve, gens, gens_p, cols, sc in test_oracle.seeded_cases(port):
+        out[f"commit{curve}"] = refcpu.commit(curve, cols, gens)
+        b = refcpu.fixed_msm(curve, gens_p, 3, 40, sc, element_num_bytes=5)
+        out[f"fixed{curve}"] = refcpu.normalize(curve, b)
+        a = port.fixed_msm(curve, gens_p, 3, 40, sc, element_num_bytes=5)
+        out[f"normalized_port_fixed{curve}"] = refcpu.normalize(curve, a)
+    np.savez_compressed(os.path.join(HERE, "oracle_cases.npz"), **out)
+
+
+def make_inner_product_seeded_fixture():
+    """tests/golden/inner_product_seeded.npz: the reference's proofs of the seeded cases of
+    tests/test_inner_product.py, from a transcript labelled b"live"."""
+    from tests import test_inner_product as tip
+    out = {"transcript_xyz": refcpu.transcript_new(b"xyz"),
+           "transcript_live": refcpu.transcript_new(b"live")}
+    for name in tip.SEEDED:
+        for key, a, b, off in tip.seeded_cases(name):
+            t = out["transcript_live"].copy()
+            lv, rv, ap = refcpu.prove_inner_product(t, a, b, off)
+            out.update({f"{key}_l": lv, f"{key}_r": rv, f"{key}_ap": ap, f"{key}_t1": t})
+    np.savez_compressed(os.path.join(HERE, "inner_product_seeded.npz"), **out)
+
+
+def _baseline_generators(curve):
+    from tests import test_gpu_baseline_sizes as t
+    af, p2 = [], []
+    for first in t.GENERATOR_SAMPLES[0]:
+        for i in t.GENERATOR_SAMPLES[1]:
+            rp2, raf = refcpu.random_elements(curve, 1, first + i)
+            af.append(raf[0])
+            p2.append(refcpu.normalize(curve, rp2)[0])
+    return {f"generators_affine{curve}": np.array(af), f"generators_normalized{curve}": np.array(p2)}
+
+
+def _baseline_c1_c2(_):
+    from tests import common, test_gpu_baseline_sizes as t
+    out = {"ristretto_generators_300_at_12345":
+           refcpu.normalize(0, refcpu.ristretto_generators(300, 12345))}
+    s = common.mt19937_bytes(0, 1 << 16)
+    out["c1"] = refcpu.commit(0, [(s, 0)], None, 0)
+    s = common.mt19937_bytes(0, 1 << 20)
+    out["c2_generators"] = np.concatenate(
+        [refcpu.normalize(0, refcpu.ristretto_generators(1, i)) for i in t.C2_GENERATOR_SAMPLES])
+    out["c2"] = refcpu.commit(0, [(s, 0)], refcpu.ristretto_generators(1 << 20, 0))
+    return out
+
+
+def _baseline_c3(_):
+    from tests import common, test_gpu_baseline_sizes as t
+    n = 1 << 18
+    s = t._scalars(n, 3, 0x7F)
+    af = refcpu.random_elements(1, n, 0)[1]
+    return {"c3": refcpu.commit(1, [(s, 0)], af),
+            "c3_closed_form": common.closed_form_commitment(refcpu, 1, s),
+            "c3_full_closed_form": common.closed_form_commitment(refcpu, 1,
+                                                                 t._scalars(1 << 22, 4, 0x7F))}
+
+
+def _baseline_c5(curve):
+    from tests import common, test_gpu_baseline_sizes as t
+    n = 1 << 18
+    af = refcpu.random_elements(curve, n, 0)[1]
+    s = t._scalars(n, 5 + curve, 0x3F)
+    bits = np.unpackbits(t.c5_packed_scalars(n), axis=1, bitorder="little")
+    cols, lo = [], 0
+    for w in t.C5_BIT_TABLE:  # the packed rows as one column per output width
+        b = np.zeros((n, 8 * ((w + 7) // 8)), dtype=np.uint8)
+        b[:, :w] = bits[:, lo:lo + w]
+        cols.append((np.packbits(b, axis=1, bitorder="little"), 0))
+        lo += w
+    out = {f"c5_{curve}": refcpu.commit(curve, [(s, 0)], af),
+           f"c5_{curve}_packed": refcpu.commit(curve, cols, af)}
+    if curve == 2:
+        out["c5_full_closed_form"] = common.closed_form_commitment(refcpu, 2,
+                                                                   t._scalars(1 << 22, 11, 0x3F))
+    return out
+
+
+def _run(job):
+    fn, arg = job
+    return fn(arg)
+
+
+def make_baseline_sizes_fixture():
+    """tests/golden/baseline_sizes.npz: the reference's results on the inputs of
+    tests/test_gpu_baseline_sizes.py (its generators at sample indices, its commitments at the
+    BASELINE sizes, one closed-form scalar multiplication for each 2^22 case)."""
+    import multiprocessing as mp
+    jobs = [(_baseline_generators, c) for c in (1, 2, 3)] + \
+        [(_baseline_c1_c2, None), (_baseline_c3, None), (_baseline_c5, 2), (_baseline_c5, 3)]
+    out = {}
+    with mp.get_context("spawn").Pool(len(jobs)) as pool:
+        for part in pool.map(_run, jobs):
+            out.update(part)
+    np.savez_compressed(os.path.join(HERE, "baseline_sizes.npz"), **out)
+
+
+def make_ref_gpu_fixture():
+    """tests/golden/ref_gpu_kernels.npz: the reference's GPU bucket kernels (oracle/_ref/
+    libblitzar_ref_gpu.so) on the inputs of tests/test_ref_gpu_kernels.py, ristretto-compressed."""
+    import blitzar_b200 as bb
+    from oracle import refgpu
+    from tests import test_ref_gpu_kernels as t
+    assert bb.sxt_init(num_precomputed_generators=64) == 0
+    out = {}
+    for n in t.SIZES:
+        gens, s = t._inputs(bb, n, seed=n)
+        p3, _, _ = refgpu.bucket_msm(gens, s)
+        out[f"n{n}"] = refcpu.normalize(0, p3)
+        assert np.array_equal(out[f"n{n}"], refcpu.commit(0, [(s, 0)], gens)), n
+    np.savez_compressed(os.path.join(HERE, "ref_gpu_kernels.npz"), **out)
+
+
+FIXTURES = {"commit": main, "inner_product": make_inner_product_fixture,
+            "oracle_cases": make_oracle_cases_fixture,
+            "inner_product_seeded": make_inner_product_seeded_fixture,
+            "baseline_sizes": make_baseline_sizes_fixture, "ref_gpu": make_ref_gpu_fixture}
+
+if __name__ == "__main__":
+    import argparse
+    ap = argparse.ArgumentParser()
+    ap.add_argument("fixtures", nargs="*", default=["commit"], choices=sorted(FIXTURES))
+    ap.add_argument("--out", default=HERE, help="directory the .npz files are written to")
+    args = ap.parse_args()
+    HERE = args.out
+    for name in args.fixtures:
+        FIXTURES[name]()

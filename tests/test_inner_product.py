@@ -1,6 +1,6 @@
 """Inner-product argument (sxt_curve25519_prove_inner_product / _verify_): byte-exact against the
-reference's cpu backend — committed fixtures generated from oracle/_ref (tests/golden/
-inner_product.npz, script make_golden.py) and, when oracle/_ref is present, live random cases.
+reference's cpu backend — committed fixtures generated from it by tests/golden/make_golden.py
+(inner_product.npz: proofs and verification; inner_product_seeded.npz: proofs of seeded_cases).
 Mirrors cbindings/inner_product_proof.t.cc (prove then verify, tampered inputs are rejected).
 The C port of the oracle restates the protocol too and is pinned on the same fixtures."""
 import os
@@ -8,7 +8,9 @@ import os
 import numpy as np
 import pytest
 
-GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "inner_product.npz")
+GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+GOLDEN = os.path.join(GOLDEN_DIR, "inner_product.npz")
+SEEDED_GOLDEN = os.path.join(GOLDEN_DIR, "inner_product_seeded.npz")
 L = 2**252 + 27742317777372353535851937790883648493
 
 
@@ -42,19 +44,36 @@ def test_oracle_port_matches_reference_fixture(port):
     _check_against_fixture(port)
 
 
-def test_oracle_port_matches_reference_live(port, refcpu):
-    rng = np.random.default_rng(15)
-    for n in (1, 2, 7, 12):
+# (rng seed, sizes, generators offset) of the seeded cases; the reference's proofs of them and its
+# transcripts are in inner_product_seeded.npz
+SEEDED = {"port": (15, (1, 2, 7, 12), 4), "emul": (5, (3, 8, 21), 2)}
+
+
+def seeded_cases(name):
+    """Yields (key, a, b, generators offset): scalars reduced mod l."""
+    seed, sizes, off = SEEDED[name]
+    rng = np.random.default_rng(seed)
+    for n in sizes:
         av = [int.from_bytes(rng.bytes(32), "little") % L for _ in range(n)]
         bv = [int.from_bytes(rng.bytes(32), "little") % L for _ in range(n)]
         a = np.array([list(v.to_bytes(32, "little")) for v in av], dtype=np.uint8)
         b = np.array([list(v.to_bytes(32, "little")) for v in bv], dtype=np.uint8)
-        assert np.array_equal(port.transcript_new(b"xyz"), refcpu.transcript_new(b"xyz"))
-        t_ref = refcpu.transcript_new(b"live")
-        t = t_ref.copy()
-        want = refcpu.prove_inner_product(t_ref, a, b, 4)
-        got = port.prove_inner_product(t, a, b, 4)
-        assert all(np.array_equal(x, y) for x, y in zip(want, got)) and np.array_equal(t, t_ref)
+        yield f"{name}{n}", a, b, off
+
+
+def _check_against_seeded(engine, name):
+    z = np.load(SEEDED_GOLDEN)
+    for key, a, b, off in seeded_cases(name):
+        t = z["transcript_live"].copy()
+        got = engine.prove_inner_product(t, a, b, off)
+        want = (z[f"{key}_l"], z[f"{key}_r"], z[f"{key}_ap"])
+        assert all(np.array_equal(x, y) for x, y in zip(want, got)), key
+        assert np.array_equal(t, z[f"{key}_t1"]), key
+
+
+def test_oracle_port_matches_reference_live(port):
+    assert np.array_equal(port.transcript_new(b"xyz"), np.load(SEEDED_GOLDEN)["transcript_xyz"])
+    _check_against_seeded(port, "port")
 
 
 def test_emulated_pipeline_matches_reference_fixture(emul):
@@ -75,18 +94,8 @@ def test_emulated_pipeline_matches_oracle_port_live(emul, port):
         assert all(np.array_equal(x, y) for x, y in zip(want, got)) and np.array_equal(t1, t2)
 
 
-def test_emulated_pipeline_matches_reference_live(emul, refcpu):
-    rng = np.random.default_rng(5)
-    for n in (3, 8, 21):
-        av = [int.from_bytes(rng.bytes(32), "little") % L for _ in range(n)]
-        bv = [int.from_bytes(rng.bytes(32), "little") % L for _ in range(n)]
-        a = np.array([list(v.to_bytes(32, "little")) for v in av], dtype=np.uint8)
-        b = np.array([list(v.to_bytes(32, "little")) for v in bv], dtype=np.uint8)
-        t_ref = refcpu.transcript_new(b"live")
-        t = t_ref.copy()
-        want = refcpu.prove_inner_product(t_ref, a, b, 2)
-        got = emul.prove_inner_product(t, a, b, 2)
-        assert all(np.array_equal(x, y) for x, y in zip(want, got)) and np.array_equal(t, t_ref)
+def test_emulated_pipeline_matches_reference_live(emul):
+    _check_against_seeded(emul, "emul")
 
 
 @pytest.mark.gpu

@@ -1,5 +1,5 @@
-"""The oracle itself: pinned against the reference's golden vector, the committed fixtures that
-were generated from the reference's own CPU implementation, and (when present) oracle/_ref live."""
+"""The oracle itself: pinned against the reference's golden vector and the committed fixtures that
+were generated from the reference's own CPU implementation (tests/golden/make_golden.py)."""
 import os
 
 import numpy as np
@@ -35,20 +35,26 @@ def test_builtin_generators_fixture(port):
     assert np.array_equal(port.normalize(0, g), z["compressed"])
 
 
-def test_port_matches_reference_live(port, refcpu):
+def seeded_cases(port):
+    """Per curve: (curve, commit generators, projective generators, columns, fixed-MSM scalars).
+    tests/golden/make_golden.py runs the reference on the same cases (oracle_cases.npz)."""
     rng = np.random.default_rng(11)
-    assert refcpu.commit(0, common.golden_columns()).tolist() == common.GOLDEN_COMMITMENTS
     for curve in range(4):
         gens, gens_p = common.generators_for(port, curve, 120)
         cols = common.random_columns(rng, 120, [(0, 32, 0), (-7, 16, 1), (0, 3, 0), (-119, 32, 0),
                                                  (-120, 8, 0)]) + common.edge_case_columns()
-        assert common.same(curve, port.commit(curve, cols, gens), refcpu.commit(curve, cols, gens))
         sc = rng.integers(0, 256, (40, 3 * 5), dtype=np.uint8)
-        a = port.fixed_msm(curve, gens_p[:40], 3, 40, sc, element_num_bytes=5)
-        b = refcpu.fixed_msm(curve, gens_p[:40], 3, 40, sc, element_num_bytes=5)
-        assert common.same(curve, port.normalize(curve, a), refcpu.normalize(curve, b))
+        yield curve, gens, gens_p[:40], cols, sc
+
+
+def test_port_matches_reference_live(port):
+    z = np.load(os.path.join(GOLDEN_DIR, "oracle_cases.npz"))
+    for curve, gens, gens_p, cols, sc in seeded_cases(port):
+        assert common.same(curve, port.commit(curve, cols, gens), z[f"commit{curve}"])
+        a = port.fixed_msm(curve, gens_p, 3, 40, sc, element_num_bytes=5)
+        assert common.same(curve, port.normalize(curve, a), z[f"fixed{curve}"])
         # the two normalisers agree on the same projective input
-        assert common.same(curve, port.normalize(curve, a), refcpu.normalize(curve, a))
+        assert common.same(curve, port.normalize(curve, a), z[f"normalized_port_fixed{curve}"])
 
 
 def test_reference_fixed_pedersen_vectors(port):

@@ -1,6 +1,8 @@
 """The reference's own GPU bucket kernels (oracle/_ref/libblitzar_ref_gpu.so, SURVEY §8c / Appendix
 B) on the same B200, same inputs: results must agree with ours, and the timings are the
-GPU-vs-GPU comparison quoted in RESULTS.md. Run as a script for the C2-size numbers:
+GPU-vs-GPU comparison quoted in RESULTS.md. The test compares with the results those kernels gave
+on its inputs, stored in tests/golden/ref_gpu_kernels.npz (tests/golden/make_golden.py ref_gpu).
+Run as a script for the C2-size numbers (needs oracle/_ref):
     python tests/test_ref_gpu_kernels.py [log2 n]"""
 import os
 import sys
@@ -13,6 +15,9 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 pytestmark = pytest.mark.gpu
 
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_gpu_kernels.npz")
+SIZES = (1, 50, 191, 193, 20000)
+
 
 def _inputs(bb, n, seed=5):
     rng = np.random.default_rng(seed)
@@ -22,14 +27,11 @@ def _inputs(bb, n, seed=5):
     return gens, s
 
 
-def test_reference_gpu_kernels_agree(bb, refcpu):
-    from oracle import refgpu
-    if not refgpu.available():
-        pytest.skip("oracle/_ref/libblitzar_ref_gpu.so not built")
-    for n in (1, 50, 191, 193, 20000):
+def test_reference_gpu_kernels_agree(bb):
+    z = np.load(GOLDEN)
+    for n in SIZES:
         gens, s = _inputs(bb, n, seed=n)
-        p3, _, _ = refgpu.bucket_msm(gens, s)
-        want = refcpu.normalize(0, p3)  # ristretto compression of the reference GPU result
+        want = z[f"n{n}"]  # ristretto compression of the reference GPU result
         got = bb.compute_pedersen_commitments(0, [(s, 0)], gens)
         assert np.array_equal(got, want), n
 
