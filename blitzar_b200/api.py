@@ -13,6 +13,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "libblitzar_b200.so")
 
 SXT_CPU_BACKEND, SXT_GPU_BACKEND = 1, 2
 SXT_CURVE_RISTRETTO255, SXT_CURVE_BLS_381, SXT_CURVE_BN_254, SXT_CURVE_GRUMPKIN = 0, 1, 2, 3
+SXT_FIELD_SCALAR255, SXT_FIELD_GRUMPKIN = 0, 1
 # per curve: (projective ABI bytes, commitment-generator stride, commitment output bytes)
 CURVE_SIZES = {0: (160, 160, 32), 1: (144, 104, 48), 2: (96, 72, 72), 3: (96, 72, 72)}
 
@@ -38,7 +39,7 @@ B200_SYMBOLS = [
     "b200_profile_read", "b200_set_reduce_groups", "b200_stream",
     "b200_synthetic_generators_device", "b200_commit_host_partials",
     "b200_fixed_msm_host_partials", "b200_multiexp_handle_new_device",
-    "b200_selftest_lane_arithmetic",
+    "b200_selftest_lane_arithmetic", "b200_prove_sumcheck_device",
 ]
 
 
@@ -384,3 +385,80 @@ def verify_inner_product(transcript, b, product, a_commit, l_vector, r_vector, a
         _ptr(transcript), C.c_uint64(n), C.c_uint64(generators_offset), _ptr(b),
         _ptr(np.ascontiguousarray(product)), _ptr(np.ascontiguousarray(a_commit)), _ptr(lv),
         _ptr(rv), _ptr(np.ascontiguousarray(ap_value))))
+
+
+# ---- sumcheck (blitzar_api.h:133-183, :766) --------------------------------------------------------
+class sumcheck_descriptor(C.Structure):
+    _fields_ = [("mles", C.c_void_p), ("product_table", C.c_void_p),
+                ("product_terms", C.POINTER(C.c_uint)), ("n", C.c_uint), ("num_mles", C.c_uint),
+                ("num_products", C.c_uint), ("num_product_terms", C.c_uint),
+                ("round_degree", C.c_uint)]
+
+
+# void (FIELD* r, void* context, const FIELD* polynomial, unsigned polynomial_len)
+SUMCHECK_CALLBACK = C.CFUNCTYPE(None, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint)
+
+
+def sumcheck_num_variables(n):
+    return max((n - 1).bit_length(), 1)
+
+
+def pack_product_table(field_id, product_table):
+    """product_table: [(multiplier as 32 ABI bytes, product_length)] -> the C layout of
+    std::pair<FIELD, unsigned>: 36-byte entries for scalar255, 40-byte entries for grumpkin (the
+    length at byte 32, padding zero)."""
+    stride = 36 if field_id == SXT_FIELD_SCALAR255 else 40
+    out = np.zeros((max(len(product_table), 1), stride), dtype=np.uint8)
+    for k, (mult, length) in enumerate(product_table):
+        out[k, :32] = np.frombuffer(bytes(mult), dtype=np.uint8)
+        out[k, 32:36] = np.frombuffer(np.uint32(length).tobytes(), dtype=np.uint8)
+    return out
+
+
+def sumcheck_args(field_id, mles_ptr, n, num_mles, product_table, product_terms, callback,
+                  round_degree=None):
+    """ctypes arguments of sxt_prove_sumcheck / b200_prove_sumcheck_device (and the emulated
+    prover). callback(polynomial uint8 [len, 32]) returns the round's challenge r as 32 ABI bytes.
+    Returns (args, polynomials [num_variables, round_degree + 1, 32], evaluation_point
+    [num_variables, 32], keepalive)."""
+    if round_degree is None:
+        round_degree = max([length for _, length in product_table], default=1)
+    v = sumcheck_num_variables(n)
+    polys = np.zeros((v, round_degree + 1, 32), dtype=np.uint8)
+    point = np.zeros((v, 32), dtype=np.uint8)
+    table = pack_product_table(field_id, product_table)
+    terms = (C.c_uint * max(len(product_terms), 1))(*product_terms)
+
+    def trampoline(r, _ctx, poly, length):
+        p = np.ctypeslib.as_array(C.cast(poly, C.POINTER(C.c_uint8)), shape=(length * 32,))
+        C.memmove(r, bytes(callback(p.reshape(length, 32).copy())), 32)
+
+    cb = SUMCHECK_CALLBACK(trampoline)
+    desc = sumcheck_descriptor(mles_ptr, table.ctypes.data, terms, n, num_mles, len(product_table),
+                               len(product_terms), round_degree)
+    args = (_ptr(polys), _ptr(point), C.c_uint(field_id), C.byref(desc), C.cast(cb, C.c_void_p),
+            C.c_void_p(None))
+    return args, polys, point, (table, terms, cb, desc)
+
+
+def prove_sumcheck(field_id, mles, product_table, product_terms, callback, round_degree=None):
+    """sxt_prove_sumcheck. mles: uint8 [num_mles, n, 32] (MLE j is mles[j], ABI form of the field);
+    product_table: [(multiplier 32 bytes, product_length)]; product_terms: MLE indices of every
+    product, concatenated; callback(polynomial uint8 [len, 32]) -> r (32 bytes).
+    Returns (polynomials [num_variables, round_degree + 1, 32], evaluation_point [num_variables, 32])."""
+    mles = np.ascontiguousarray(mles, dtype=np.uint8)
+    args, polys, point, _keep = sumcheck_args(field_id, mles.ctypes.data, mles.shape[1],
+                                              mles.shape[0], product_table, product_terms,
+                                              callback, round_degree)
+    lib().sxt_prove_sumcheck(*args)
+    return polys, point
+
+
+def prove_sumcheck_device(field_id, mles_ptr, n, num_mles, product_table, product_terms, callback,
+                          round_degree=None):
+    """b200_prove_sumcheck_device: as prove_sumcheck with the MLEs already in HBM (device pointer,
+    the same column-major layout)."""
+    args, polys, point, _keep = sumcheck_args(field_id, mles_ptr, n, num_mles, product_table,
+                                              product_terms, callback, round_degree)
+    lib().b200_prove_sumcheck_device(*args)
+    return polys, point

@@ -12,7 +12,8 @@ LIB = os.path.join(LIBDIR, "libblitzar_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC"]
-UNITS = ["api.cu", "curve_ed25519.cu", "curve_bls12381.cu", "curve_bn254.cu", "curve_grumpkin.cu"]
+UNITS = ["api.cu", "curve_ed25519.cu", "curve_bls12381.cu", "curve_bn254.cu", "curve_grumpkin.cu",
+         "sumcheck.cu"]
 
 
 def _newer(target, sources):
@@ -61,8 +62,8 @@ def build_emul():
     prefix = os.path.join(edir, "emul_prefix.h")
     flags = ["g++", "-std=c++17", "-O1", "-DB200_EMULATE", "-fPIC", "-w", "-include", prefix]
     jobs, objs = [], []
-    for u in [x for x in UNITS if x.startswith("curve_")] + ["emul.cpp"]:
-        src = os.path.join(edir if u == "emul.cpp" else CSRC, u)
+    for u in [x for x in UNITS if x.startswith("curve_")] + ["emul.cpp", "emul_sumcheck.cpp"]:
+        src = os.path.join(edir if u.startswith("emul") else CSRC, u)
         obj = os.path.join(objdir, u.rsplit(".", 1)[0] + ".o")
         objs.append(obj)
         if _newer(obj, [src, prefix] + _headers()):
@@ -91,7 +92,9 @@ def build_oracle_ref():
     oracle/_ref/libblitzar_ref_cpu.so that travels with the snapshot."""
     if not os.path.isdir("/root/reference/sxt"):
         return None
-    subprocess.check_call(["make", "-s", "-j8", "-C", os.path.join(ROOT, "oracle", "ref_build")],
+    ref_build = os.path.join(ROOT, "oracle", "ref_build")
+    subprocess.check_call(["make", "-s", "-j8", "-C", ref_build], stdout=subprocess.DEVNULL)
+    subprocess.check_call(["make", "-s", "-f", os.path.join(ref_build, "sumcheck.mk")],
                           stdout=subprocess.DEVNULL)
     return os.path.join(ROOT, "oracle", "_ref", "libblitzar_ref_cpu.so")
 

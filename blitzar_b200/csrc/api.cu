@@ -959,9 +959,15 @@ int sxt_curve25519_verify_inner_product(struct sxt_transcript* transcript, uint6
                     reinterpret_cast<const uint8_t*>(l_vector),
                     reinterpret_cast<const uint8_t*>(r_vector), ap_value->bytes);
 }
-void sxt_prove_sumcheck(void*, void*, unsigned, const struct sumcheck_descriptor*, void*, void*) {
-  die("sxt_prove_sumcheck is not provided by blitzar_b200 (MSM hot path only)", __FILE__,
-      __LINE__);
+// blitzar_api.h:766 — as cpu_backend.cc:73-112 / gpu_backend.cc:106-145; the callback runs with the
+// library mutex held
+void sxt_prove_sumcheck(void* polynomials, void* evaluation_point, unsigned field_id,
+                        const struct sumcheck_descriptor* descriptor, void* transcript_callback,
+                        void* transcript_context) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  require_init("sxt_prove_sumcheck");
+  sumcheck_prove(ctx(), polynomials, evaluation_point, field_id, descriptor, transcript_callback,
+                 transcript_context, false);
 }
 
 struct sxt_multiexp_handle* sxt_multiexp_handle_new(unsigned curve_id, const void* generators,
@@ -1238,6 +1244,14 @@ void b200_synthetic_generators_device(unsigned curve_id, void* out_generators, u
   require_init("b200_synthetic_generators_device");
   B200_REQUIRE(out_generators != nullptr, "out_generators == nullptr");
   vt(curve_id).synth_generators(ctx(), out_generators, n, first, projective != 0);
+}
+void b200_prove_sumcheck_device(void* polynomials, void* evaluation_point, unsigned field_id,
+                                const struct sumcheck_descriptor* descriptor,
+                                void* transcript_callback, void* transcript_context) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  require_init("b200_prove_sumcheck_device");
+  sumcheck_prove(ctx(), polynomials, evaluation_point, field_id, descriptor, transcript_callback,
+                 transcript_context, true);
 }
 unsigned b200_selftest_lane_arithmetic(unsigned warps, unsigned seed) {
   std::lock_guard<std::mutex> lock(g_mutex);

@@ -140,6 +140,12 @@ int ipa_verify(const EngineCtx& ctx, uint8_t* transcript203, uint64_t n,
                const uint8_t* a_commit160, const uint8_t* l_vector, const uint8_t* r_vector,
                const uint8_t* ap_value);
 
+// sumcheck prover (sumcheck.cuh); the contract of sxt_prove_sumcheck, descriptor->mles a device
+// pointer when mles_on_device. Aborts with a message on an invalid descriptor.
+void sumcheck_prove(const EngineCtx& ctx, void* polynomials, void* evaluation_point,
+                    unsigned field_id, const sumcheck_descriptor* descriptor,
+                    void* transcript_callback, void* transcript_context, bool mles_on_device);
+
 // lane-sliced field arithmetic self-test (lanefield.cuh): number of mismatching checks over
 // `warps` warps of pseudo-random / edge-case operands
 unsigned selftest_lane_arithmetic(const EngineCtx& ctx, unsigned warps, unsigned seed);
